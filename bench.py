@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/s of the Deformable-DETR R50 hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one training pass of the hot path over one synthetic batch per GPU:
@@ -108,6 +108,25 @@ def dense_flops_per_step(step_fn):
         return None
     finally:
         fl._TCGEN05 = own
+
+
+DUMP_PARAM_SAMPLE = 1 << 22
+
+
+def dump_outputs(out_dir, loss, model):
+    """Write what the last timed step handed its caller: loss.npy, and params.npy with the trainable parameters as that
+    step's optimizer update left them (the flat optimizer zeroes the gradient once it has used it).  The parameters are
+    taken in model order, whatever their memory layout, and a fixed seeded sample of 4 M of them is written (16 MB).
+    Inputs, initial weights and dropout masks are seeded, but the step's atomic reductions and autotuned cuDNN algorithms
+    are not bit-reproducible, and the optimizer compounds that over the warm-up and timed steps: compare two builds
+    against the spread of two runs of one build, not bit for bit."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    flat = torch.cat([p.detach().reshape(-1) for p in model.parameters() if p.requires_grad]).float()
+    n = min(flat.numel(), DUMP_PARAM_SAMPLE)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+    np.save(os.path.join(out_dir, "params.npy"), flat[idx.to(flat.device)].cpu().numpy())
 
 
 def golden_parity(dev):
@@ -331,14 +350,21 @@ def c5_arm(args, rank, local_rank, world):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
+    last = {}
+
+    def timed_step():
+        last["loss"] = step(dev_frames)
+
     if sampler:
         sampler.mark_begin()
     l0 = msda.launch_count()
-    ms_total = timed(lambda: step(dev_frames))
+    ms_total = timed(timed_step)
     launches = msda.launch_count() - l0
     if sampler:
         sampler.mark_end()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["loss"], model)
     ms_e2e = timed(lambda: float(step(host.to(dev, non_blocking=True)).item()))
     if rank == 0:
         line = {"metric": "frames/sec TrackFormer multi-frame train step 1080x1920 (BASELINE configs[4])",
@@ -398,7 +424,13 @@ def main():
                          "previous frame (eager: the track-query injection draws from the host RNG, like the reference)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arms, not to --impl reference")
     _claim_stdout()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -509,13 +541,20 @@ def main():
         return
 
     # (1) device-resident throughput
+    last = {}
+
+    def timed_step():
+        last["loss"] = step(dev_frames, targets)
+
     if sampler:
         sampler.mark_begin()
-    ms_total = timed(lambda: step(dev_frames, targets), args.steps)
+    ms_total = timed(timed_step, args.steps)
     if sampler:
         sampler.mark_end()
     clocks = sampler.stop() if sampler else None
     value = bpg * world * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:                 # before the regions below move the model on
+        dump_outputs(args.dump_outputs, last["loss"], model)
 
     # (2) end to end: pinned host frame -> device every step, loss read back every step
     #     The copy of step i + 1's frame is started (TrainStep.prefetch: side stream, staging buffer) right after step i

@@ -33,6 +33,35 @@ def test_reference_arm_runs_on_rank_zero_only():
     assert r.returncode == 0 and r.stdout == ""
 
 
+def test_dump_outputs_writes_loss_and_a_fixed_parameter_sample(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    model = torch.nn.Sequential(torch.nn.Linear(4, 3), torch.nn.Linear(3, 2))
+    model[0].bias.requires_grad_(False)
+    trainable = torch.cat([p.detach().reshape(-1) for p in model.parameters() if p.requires_grad]).numpy()
+    bench.dump_outputs(str(tmp_path / "all"), torch.tensor(1.5), model)
+    loss = np.load(tmp_path / "all" / "loss.npy")
+    assert loss.dtype == np.float32 and loss.shape == () and loss == 1.5
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "params.npy"), trainable)   # small model: all, model order
+    monkeypatch.setattr(bench, "DUMP_PARAM_SAMPLE", 7)
+    runs = []
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), torch.tensor(1.5), model)
+        runs.append(np.load(tmp_path / d / "params.npy"))
+    assert runs[0].dtype == np.float32 and runs[0].shape == (7,)
+    np.testing.assert_array_equal(runs[0], runs[1])                                      # same positions every run
+    pos = [int(np.flatnonzero(trainable == v)[0]) for v in runs[0]]
+    assert pos == sorted(pos)
+
+
+def test_steps_must_be_positive_and_dump_needs_the_cuda_arm():
+    r = _run(["--impl", "reference", "--steps", "0"])
+    assert r.returncode != 0 and "--steps" in r.stderr
+    r = _run(["--impl", "reference", "--steps", "1", "--dump-outputs", "unused"])
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+
+
 def test_product_arm_fails_loudly_without_a_gpu():
     import torch
     if torch.cuda.is_available():
